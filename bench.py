@@ -49,6 +49,7 @@ WORKLOADS = {
                           label="BigVGAN-large 24kHz", config="config 5 (per-GPU shard: 32 of 256 utterances)"),
 }
 N_MEL = 80   # kept for scripts that import it
+DUMP_BYTES = 32 << 20   # --dump-outputs: the full config-2 waveform is 64 MiB, half of its utterances are kept
 
 
 def parse():
@@ -64,7 +65,31 @@ def parse():
     ap.add_argument("--no-also", action="store_true", help="only the headline workload (quick iteration)")
     ap.add_argument("--workload", default="hifigan_v1", choices=list(WORKLOADS),
                     help="headline workload of the line; hifigan_v1 = BASELINE config 2 (default)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the waveform the headline workload's last timed step returned "
+                         "as DIR/wav.npy (float32; beyond %d MiB a fixed seeded sample of its utterances)" % (DUMP_BYTES >> 20))
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs writes the native path's outputs")
+    return args
+
+
+def dump_output(out_dir, name, wav):
+    """Write a generator output [B, 1, N] as out_dir/<name>.npy in float32.  If it is larger than DUMP_BYTES, keep
+    the utterances of a fixed seeded draw (in batch order) and, should one utterance alone exceed the budget, its
+    leading samples: two builds run with the same arguments then write the same selection."""
+    import numpy as np
+    import torch
+    B, N = wav.shape[0], wav[0].numel()
+    rows = min(B, max(1, DUMP_BYTES // (4 * N)))
+    cols = min(N, DUMP_BYTES // (4 * rows))
+    if rows < B:
+        idx = torch.randperm(B, generator=torch.Generator().manual_seed(0))[:rows].sort().values
+        wav = wav[idx.to(wav.device)]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, name + ".npy"), wav[..., :cols].float().cpu().numpy())
 
 
 def make_cfg(workload="hifigan_v1"):
@@ -277,9 +302,11 @@ def _roofline(prof, ms_total, samples_rank_step, flop, workload, B, T, precision
     return r
 
 
-def measure_generator(workload, args, dev, rank, world, steps, warmup, want_cpu, clocks_on_rank0=True, shape=None):
+def measure_generator(workload, args, dev, rank, world, steps, warmup, want_cpu, clocks_on_rank0=True, shape=None,
+                      dump_dir=None):
     """One workload on the native path: device-resident `value` (CUDA events, max over ranks), `e2e` through the
-    reference-facing call with pinned host buffers, per-class roofline from the C ABI's launch events."""
+    reference-facing call with pinned host buffers, per-class roofline from the C ABI's launch events.  With
+    `dump_dir`, the output of the last timed step is written there (dump_output)."""
     import torch
     import torch.distributed as dist
     from amphion_b200.dist import sharded_vocoder_inference, _sharded_forward
@@ -327,8 +354,9 @@ def measure_generator(workload, args, dev, rank, world, steps, warmup, want_cpu,
         barrier(); torch.cuda.synchronize()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        for _ in range(steps):
+        for _ in range(steps - 1):
             step()
+        last = step()
         e1.record()
         torch.cuda.synchronize(); barrier()
         ms_total = e0.elapsed_time(e1)
@@ -336,6 +364,9 @@ def measure_generator(workload, args, dev, rank, world, steps, warmup, want_cpu,
         model.set_profiling(False)
         clocks = sampler.stop() if (rank == 0 and clocks_on_rank0) else None
         launches = model.last_launches * steps * world      # whole job (every rank runs the same pipeline)
+        if dump_dir is not None and last is not None:       # ranks other than the gather's destination hold None
+            dump_output(dump_dir, "wav", last)
+        del last
 
         # ---- end to end through the reference-facing call, host buffers in, host result out ----
         mel_host = mel.cpu().pin_memory()
@@ -519,7 +550,8 @@ def run_native(args, rank, local_rank, world):
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
     want_cpu = world == 1 and not args.no_cpu_baseline
-    main = measure_generator(args.workload, args, dev, rank, world, args.steps, args.warmup, want_cpu)
+    main = measure_generator(args.workload, args, dev, rank, world, args.steps, args.warmup, want_cpu,
+                             dump_dir=args.dump_outputs)
     also, eager = {}, None
     if not args.no_also and not os.environ.get("AB_BENCH_PROFILE"):
         if world == 1:

@@ -1,3 +1,4 @@
+import hashlib
 import os
 import sys
 
@@ -62,6 +63,40 @@ GOLDEN_APNET = (dict(ASP_channel=32, ASP_resblock_kernel_sizes=[3, 7, 11], ASP_r
                      PSP_channel=48, PSP_resblock_kernel_sizes=[3, 7], PSP_resblock_dilation_sizes=[[1, 3, 5], [1, 2, 4]],
                      PSP_input_conv_kernel_size=5, PSP_output_R_conv_kernel_size=7, PSP_output_I_conv_kernel_size=7),
                 dict(n_mel=12, n_fft=64, hop_size=16, win_size=64, extract_amplitude_phase=True, sample_rate=16000))
+
+
+def state_dict_sha256(keys, sd):
+    """Digest of a state dict: every key, its shape and its float32 bytes, in the given order."""
+    h = hashlib.sha256()
+    for k in keys:
+        v = np.ascontiguousarray(sd[k], dtype=np.float32)
+        h.update(f"{k}{v.shape}".encode())
+        h.update(v.tobytes())
+    return h.hexdigest()
+
+
+def load_golden_apnet():
+    """apnet.npz keeps the reference's inputs, outputs, state-dict key order and the SHA-256 of its weights; the
+    weights themselves (1.2 MB of random initialisation) are drawn again.  APNet built under torch.manual_seed(77)
+    draws the reference's initial weights (same construction order), and the output convolutions are then rescaled
+    as gen_golden.py:gen_apnet did; the digest pins the result to the weights the reference ran with."""
+    from types import SimpleNamespace as NS
+    import torch
+    from amphion_b200.vocoders import APNet
+    g, _ = load_golden("apnet")
+    hp, pre = GOLDEN_APNET
+    torch.manual_seed(77)
+    model = APNet(NS(preprocess=NS(**pre), model=NS(generator="apnet", apnet=NS(**hp))))
+    gen = torch.Generator().manual_seed(78)
+    with torch.no_grad():
+        for conv, gain in ((model.ASP_output_conv, 3.0), (model.PSP_output_R_conv, 20.0), (model.PSP_output_I_conv, 20.0)):
+            conv.weight_g.mul_(gain)
+            conv.bias.copy_(torch.randn(conv.bias.shape, generator=gen) * 0.3)
+    own = {k: v.numpy().copy() for k, v in model.state_dict().items()}
+    keys = [str(k) for k in g.pop("sd_keys")]
+    assert list(own) == keys, "APNet state-dict keys differ from the reference's"
+    assert state_dict_sha256(keys, own) == str(g.pop("sd_sha256")), "APNet(seed 77) no longer draws the reference's weights"
+    return g, own
 
 
 # HiFiGAN_vits fixtures (positional constructor; tests/golden/gen_golden.py:gen_hifigan_vits)

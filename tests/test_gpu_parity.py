@@ -975,10 +975,10 @@ def test_apnet_matches_reference_fixture(precision, tol):
     """fp32 arithmetic reproduces the reference to 5e-5.  With 16-bit conv operands the log-amplitude and the (R, I)
     pair carry ~1e-3 of rounding, which exp() and atan2 turn into ~1e-3 RELATIVE error of the spectrum: the audio
     bound is 2e-3 (measured 1e-3-class), stated here rather than hidden."""
-    from conftest import GOLDEN_APNET
+    from conftest import GOLDEN_APNET, load_golden_apnet
     from amphion_b200.vocoders.gan_vocoder_inference import vocoder_inference
     hp, pre = GOLDEN_APNET
-    g, sd = load_golden("apnet")
+    g, sd = load_golden_apnet()
     model = _apnet_model(hp, pre, sd)
     model.precision = precision
     logamp, pha, rea, imag, audio = model(torch.from_numpy(g["mel"]).to(DEV))

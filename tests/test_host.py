@@ -5,6 +5,8 @@ back to the CPU."""
 import ctypes as C
 import os
 import re
+import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -180,9 +182,13 @@ def test_wav_writer_roundtrip(tmp_path):
     with wave.open(str(tmp_path / "a.wav")) as f:
         assert (f.getnchannels(), f.getsampwidth(), f.getframerate(), f.getnframes()) == (1, 2, 24000, 11)
         np.testing.assert_array_equal(np.frombuffer(f.readframes(11), "<i2"), x)
-    from amphion_b200.io import save_audio
-    with pytest.raises(RuntimeError):                    # no CPU fallback: the quantiser only exists as a CUDA kernel
-        save_audio(tmp_path / "b.wav", np.zeros(16, np.float32), 16000)
+    # no CPU fallback: the quantiser only exists as a CUDA kernel, so where no device is visible save_audio raises
+    # (checked in a child process with every device hidden, so that it holds on a GPU machine as well)
+    code = ("import sys; import numpy as np; from amphion_b200.io import save_audio\n"
+            "try:\n    save_audio(sys.argv[1], np.zeros(16, np.float32), 16000)\nexcept RuntimeError:\n    sys.exit(3)\n")
+    r = subprocess.run([sys.executable, "-c", code, str(tmp_path / "b.wav")], cwd=ROOT,
+                       env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
+    assert r.returncode == 3 and not (tmp_path / "b.wav").exists()
 
 
 @pytest.mark.parametrize("tag,seed", [("a", 51), ("b", 52)])
@@ -321,10 +327,10 @@ def test_apnet_state_dict_matches_the_reference_layout():
     """Keys, order and shapes of APNet's state dict equal the reference module's (fixture made from
     models/vocoders/gan/generator/apnet.py), so its checkpoints load unchanged."""
     from types import SimpleNamespace as NS
-    from conftest import GOLDEN_APNET
+    from conftest import GOLDEN_APNET, load_golden_apnet
     from amphion_b200.vocoders import APNet, _vocoders
     hp, pre = GOLDEN_APNET
-    g, sd = load_golden("apnet")
+    g, sd = load_golden_apnet()
     model = APNet(NS(preprocess=NS(**pre), model=NS(generator="apnet", apnet=NS(**hp))))
     assert _vocoders["apnet"] is APNet
     own = model.state_dict()

@@ -3,7 +3,7 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import GOLDEN_APNET, GOLDEN_MODELS, GOLDEN_NSF, GOLDEN_VITS, load_golden, load_golden_vits
+from conftest import GOLDEN_APNET, GOLDEN_MODELS, GOLDEN_NSF, GOLDEN_VITS, load_golden, load_golden_apnet, load_golden_vits
 from oracle import generator as og
 from oracle import io as oio
 from oracle import mel as om
@@ -172,7 +172,7 @@ def test_apnet_oracle_matches_reference():
     """oracle.generator.apnet_forward / istft_same against APNet.forward of the reference (apnet.py:357-399)."""
     from oracle import generator as og
     hp, pre = GOLDEN_APNET
-    g, sd = load_golden("apnet")
+    g, sd = load_golden_apnet()
     logamp, pha, rea, imag, audio = og.apnet_forward(sd, hp, g["mel"], pre["n_fft"], pre["hop_size"], pre["win_size"])
     np.testing.assert_allclose(logamp, g["logamp"], atol=2e-5)
     np.testing.assert_allclose(rea, g["rea"], atol=2e-4, rtol=1e-4)
